@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # espnet_b200 CUDA path
   python bench.py --impl reference --gpus N --steps K ...  # the reference's own CPU Speech2Text (oracle/_ref) on the host cores
+  python bench.py ... --dump-outputs DIR                   # also write the last timed step's hypotheses as DIR/*.npy
 
 A "step" is one pass of the hot path over one batch of synthetic 16 kHz waveforms: BASELINE.json configs[1],
 Conformer-large (12L/512d/8h, ff 2048, conv2d, macaron, rel-pos latest, kernel 31) + 6L Transformer decoder,
@@ -258,26 +259,20 @@ def measured_peaks():
 # ----------------------------------------------------------------------------------------------- reference arm (CPU)
 def run_reference(args, rank, world):
     """Reference arm: one step = REF_WORKERS utterances of the workload decoded concurrently by the reference's own CPU Speech2Text
-    (a bounded sample of the 64-utterance batch).  value = utterances / wall time.  A CPU decode needs one warm-up, not W: min(W, 1)
-    are run.  ESPB_REF_BUDGET_S (default 330) bounds the run: if the next timed step would overrun it, the run stops and reports the
-    steps it completed (stated in the line)."""
+    (a bounded sample of the 64-utterance batch).  value = utterances / wall time over exactly --steps timed steps.  A CPU decode needs
+    one warm-up, not W: min(W, 1) are run."""
     if rank != 0:
         return
     cfg, secs, batch, beam, ctcw, mlr = WORKLOADS[args.workload]
     workers = ref_workers()
-    t_start = time.perf_counter()
     pool = RefPool(cfg, beam, ctcw, mlr, workers, args.workload)
     warm = min(args.warmup, 1)
     waves = waveforms((warm + args.steps) * workers, secs * 16000)
-    budget = float(os.environ.get("ESPB_REF_BUDGET_S", 330))
     k = 0
     for i in range(warm):
         pool.decode(list(waves[k:k + workers])); k += workers
     walls = []
     for i in range(args.steps):
-        est = max(walls) if walls else 0.0
-        if walls and (time.perf_counter() - t_start) + est > budget:
-            break
         w, _ = pool.decode(list(waves[k:k + workers])); k += workers
         walls.append(w)
     pool.close()
@@ -293,8 +288,7 @@ def run_reference(args, rank, world):
         "config": {"workload": args.workload, "sample": "per step: " + desc, "beam": beam, "global_batch": batch,
                    "ctc_weight": ctcw, "maxlenratio": mlr, "utt_seconds": secs, "vocab": cfg["vocab"],
                    "steps_requested": args.steps, "warmup_requested": args.warmup,
-                   "note": (f"stopped after {done} of {args.steps} steps (ESPB_REF_BUDGET_S={budget:.0f} s)" if done < args.steps else "all requested steps timed")
-                           + "; a CPU decode needs no more than one warm-up"},
+                   "note": "a CPU decode needs no more than one warm-up"},
         "cpu_baseline": {"value": ups, "unit": "utterances/s", "cores": workers * REF_THREADS, "kind": ref_kind(),
                          "sample": f"{done} steps, each: {desc}; {warm} warm-up"},
         "e2e": {"value": ups, "unit": "utterances/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
@@ -399,6 +393,36 @@ def run_streaming(args, rank, local_rank, world):
             "e2e": {"value": val, "unit": "audio-s/s", "h2d_bytes_per_step": w["streams"] * w["push"] * w["pushes_per_step"] * 4, "d2h_bytes_per_step": 0},
             "gpu_launches": ops.launch_counter[0], "clocks": clocks}
     print(json.dumps(line), flush=True)
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, results, nbest):
+    """Write what BatchBeamSearch.forward_batch returned (per utterance, its hypotheses sorted best first) as float64 arrays, the top
+    `nbest` of each utterance: hyp_yseq (U, nbest, L) padded with -1, hyp_score (U, nbest) and hyp_score_<scorer> per scorer, NaN where an
+    utterance has fewer hypotheses.  Inputs are seeded, so two builds run with the same arguments can be compared array by array."""
+    import numpy as np
+
+    U = len(results)
+    L = max((len(h.yseq) for hyps in results for h in hyps[:nbest]), default=0)
+    keys = sorted({k for hyps in results for h in hyps[:nbest] for k in h.scores})
+    arrays = {"hyp_yseq": np.full((U, nbest, L), -1.0), "hyp_score": np.full((U, nbest), np.nan)}
+    arrays.update({f"hyp_score_{k}": np.full((U, nbest), np.nan) for k in keys})
+    for u, hyps in enumerate(results):
+        for j, h in enumerate(hyps[:nbest]):
+            y = h.yseq.tolist()
+            arrays["hyp_yseq"][u, j, :len(y)] = y
+            arrays["hyp_score"][u, j] = float(h.score)
+            for k, v in h.scores.items():
+                arrays[f"hyp_score_{k}"][u, j] = float(v)
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    return sorted(arrays)
 
 
 def run_b200(args, rank, local_rank, world):
@@ -558,6 +582,7 @@ def run_b200(args, rank, local_rank, world):
     barrier()
     wall = time.perf_counter() - wall0
     launches = ops.launch_counter[0]
+    res_resident = res
     dev_ms = sum(a.elapsed_time(b) for a, b in ev)
     # ---- timed: K end-to-end steps (one event pair around all of them: consecutive steps overlap copy and compute)
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -569,6 +594,7 @@ def run_b200(args, rank, local_rank, world):
     e2e_ms = e0.elapsed_time(e1)
     clocks = sampler.stop()
     n_hyp_tokens = sum(len(r[0][2]) for r in res if r)
+    dumped = dump_outputs(args.dump_outputs, res_resident, beam) if args.dump_outputs and rank == 0 else None
 
     # ---- roofline of the dominant kernel (tcgen05 3xTF32 GEMM): per-launch CUDA events over one extra step
     ops.gemm_profile = []
@@ -652,6 +678,7 @@ def run_b200(args, rank, local_rank, world):
                 "hyp_tokens_last_step": n_hyp_tokens},
         "gpu_launches": launches,
         "clocks": clocks,
+        **({"dumped_outputs": {"dir": args.dump_outputs, "arrays": dumped, "step": "last timed resident step (encode + search)"}} if dumped else {}),
         "roofline": {"bound": "tensor", "kernel": "gemm_tf32x3_2cta_kernel (all its launches in one step: encoder, CTC head, decoder memory)", "achieved": ach, "peak": peak_tf,
                      "unit": "TFLOP/s", "frac": ach / peak_tf if peak_tf else None, "traffic": NCU_TRAFFIC["dram_bytes"], "traffic_launch": NCU_TRAFFIC,
                      "peak_source": peak_src,
@@ -708,7 +735,13 @@ def main():
     ap.add_argument("--trace", action="store_true", help="CUPTI activity trace of one step (kernel durations inside the CUDA graphs) -> stderr")
     ap.add_argument("--breakdown", action="store_true", help="time every launch of one step with CUDA events and print a per-kernel table")
     ap.add_argument("--profile-one-step", action="store_true", help="warm up, then run one step inside cudaProfilerStart/Stop and exit")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the hypotheses of the last timed step (rank 0's "
+                    "utterances, top `beam` per utterance) as DIR/<name>.npy in float64")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.workload in STREAMING):
+        ap.error("--dump-outputs is implemented for the espnet_b200 arm of the non-streaming workloads")
     rank, local_rank, world = int(os.environ.get("RANK", 0)), int(os.environ.get("LOCAL_RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
     if args.impl == "reference":
         run_reference(args, rank, world)

@@ -48,3 +48,24 @@ def test_workload_tables_and_ncu_summary_parser(tmp_path, monkeypatch):
     bench._load_ncu_traffic()
     t = bench.NCU_TRAFFIC
     assert abs(t["dram_bytes"] - 1.75e9) < 1 and t["gpu_time_us_under_ncu"] == 500.5 and t["tensor_pipe_active_pct"] == 77.7 and "r02" in t["source"]
+
+
+def test_dump_outputs_layout(tmp_path):
+    """--dump-outputs: the top `nbest` hypotheses per utterance as float64 arrays, padded with -1 (tokens) / NaN (scores)."""
+    import numpy as np
+    import torch
+
+    sys.path.insert(0, ROOT)
+    import bench
+    from espnet_b200.search import Hypothesis
+
+    res = [[Hypothesis(yseq=torch.tensor([9, 3, 4, 9]), score=-1.5, scores={"decoder": -1.0, "ctc": -2.5}),
+            Hypothesis(yseq=torch.tensor([9, 9]), score=-3.0, scores={"decoder": -2.0, "ctc": -5.0}),
+            Hypothesis(yseq=torch.tensor([9, 5, 9]), score=-4.0, scores={"decoder": -3.0, "ctc": -7.0})], []]
+    names = bench.dump_outputs(str(tmp_path / "out"), res, 2)
+    assert names == ["hyp_score", "hyp_score_ctc", "hyp_score_decoder", "hyp_yseq"]
+    a = {n: np.load(tmp_path / "out" / f"{n}.npy") for n in names}
+    assert all(v.dtype == np.float64 for v in a.values())
+    np.testing.assert_array_equal(a["hyp_yseq"], [[[9, 3, 4, 9], [9, 9, -1, -1]], [[-1] * 4] * 2])
+    np.testing.assert_array_equal(a["hyp_score"], [[-1.5, -3.0], [np.nan, np.nan]])
+    np.testing.assert_array_equal(a["hyp_score_ctc"], [[-2.5, -5.0], [np.nan, np.nan]])

@@ -1,8 +1,14 @@
-"""The reference's scorer protocol (espnet2/legacy/nets/scorer_interface.py:85-188) on the espnet_b200 classes, driven by the REFERENCE's own
-BatchBeamSearch (unmodified files under oracle/_ref): TransformerDecoder.batch_score / select_state and CTCPrefixScorer.batch_init_state /
-batch_score_partial / select_state must reproduce the n-best lists the reference produced with its own scorers (tests/golden/*.npz).
-CPU: C-ABI entry points emulated (tests/emu_backend.py) -> host logic of the protocol; GPU (-m gpu): the CUDA kernels, plus the registry path
-(espnet_b200.integration.register + the reference's own Speech2Text on device="cuda")."""
+"""The reference's scorer protocol (espnet2/legacy/nets/scorer_interface.py:85-188) on the espnet_b200 classes.
+
+Replay: tests/golden/scorer_replay.npz (tests/golden/make_golden_scorer_replay.py) holds every call the REFERENCE's own BatchBeamSearch made
+into its own TransformerDecoder and CTCPrefixScorer while decoding the tiny / small fixtures: batch_init_state, batch_score /
+batch_score_partial with the prefixes, candidate ids and the states it threads through, select_state with its index arguments,
+final_score.  TransformerDecoder.batch_score / select_state and CTCPrefixScorer.batch_init_state / batch_score_partial / select_state
+receive the same call sequence and must return the scores the reference's scorers returned.
+CPU: C-ABI entry points emulated (tests/emu_backend.py) -> host logic of the protocol; GPU (-m gpu): the CUDA kernels.
+Registry path (-m gpu, needs the reference's own files under oracle/_ref): espnet_b200.integration.register + the reference's own
+Speech2Text on device="cuda"."""
+import json
 import os
 import sys
 
@@ -10,7 +16,7 @@ import numpy as np
 import pytest
 import torch
 
-from golden_util import decode_params, decode_results, load
+from golden_util import GOLDEN_DIR, decode_params, decode_results, load
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -30,39 +36,52 @@ def _reference():
     install_ref.activate()
 
 
-def _ref_search(model, z, dn, ctc_scorer, decoder):
-    """espnet2.bin.asr_inference.Speech2Text.__init__'s BatchBeamSearch wiring (asr_inference.py:168-176, 310-381) with our scorers."""
-    from espnet2.legacy.nets.batch_beam_search import BatchBeamSearch
-    from espnet2.legacy.nets.scorers.length_bonus import LengthBonus
+def _replay(model, case, dn, device):
+    """Drive our decoder / CTC scorer through the reference search's recorded calls; compare every score matrix they return."""
+    from espnet_b200 import CTCPrefixScorer
 
-    kw = decode_params(z, dn)
-    cw = kw["ctc_weight"]
-    V = model.vocab_size
-    scorers = dict(decoder=decoder, ctc=ctc_scorer, length_bonus=LengthBonus(V))
-    weights = dict(decoder=1.0 - cw, ctc=cw, lm=1.0, ngram=0.9, length_bonus=kw.get("penalty", 0.0))
-    bs = BatchBeamSearch(beam_size=kw["beam_size"], weights=weights, scorers=scorers, sos=model.sos, eos=model.eos, vocab_size=V,
-                         token_list=model.token_list, pre_beam_score_key=None if cw == 1.0 else "full",
-                         normalize_length=kw.get("normalize_length", False))
-    return bs, kw
+    rec = np.load(os.path.join(GOLDEN_DIR, "scorer_replay.npz"))
+    log = json.loads(str(rec[f"{case}:{dn}:log"]))
+    x = torch.from_numpy(load(case)[0]["enc"]).to(device)
+    scorers = dict(decoder=model.decoder, ctc=CTCPrefixScorer(model.ctc, model.eos))
+    states = {}
 
+    def t(key):
+        return torch.from_numpy(rec[key]).to(device)
 
-def _check(hyps, gold):
-    assert len(hyps) >= len(gold)
-    for h, (yseq, score, _) in zip(hyps, gold):
-        assert h.yseq.tolist() == yseq
-        assert abs(float(h.score) - score) <= 2e-4 * max(1.0, abs(score))
+    def get(h):   # a recorded handle, a list of per-hypothesis handles, or None
+        return [states[v] for v in h] if isinstance(h, list) else (None if h is None else states[h])
 
+    def put(h, v):
+        if isinstance(h, list):
+            assert len(h) == len(v)
+            states.update(zip(h, v))
+        else:
+            states[h] = v
 
-def _drive(model, z, dn, device):
-    from espnet_b200 import integration
-
-    enc = torch.from_numpy(z["enc"]).to(device)
-    dec = integration.register()["decoder"]["b200_transformer"]
-    decoder = model.decoder
-    decoder.__class__ = dec      # same weights, now an instance of AbsDecoder + BatchScorerInterface (a subclass of its former class)
-    bs, kw = _ref_search(model, z, dn, integration.ctc_prefix_scorer(model.ctc, model.eos), decoder)
-    hyps = bs(x=enc, maxlenratio=kw.get("maxlenratio", 0.0), minlenratio=kw.get("minlenratio", 0.0))
-    _check(hyps[:10], decode_results(z, dn))
+    for n, c in enumerate(log):
+        d, what = scorers[c["scorer"]], f"call {n}: {c['scorer']}.{c['op']}"
+        if c["op"] == "init":
+            put(c["out"], d.batch_init_state(x))
+            continue
+        if c["op"] == "select":
+            s = get(c["state"])
+            put(c["out"], d.select_state(s, c["i"]) if c["new_id"] is None else d.select_state(s, c["i"], c["new_id"]))
+            continue
+        if c["op"] == "final":
+            assert d.final_score(get(c["state"])) == c["value"], what
+            continue
+        ys = t(c["ys"])
+        if c["op"] == "score":
+            scores, new = d.batch_score(ys, get(c["state"]), x.expand(ys.shape[0], *x.shape))
+            new = list(new)
+        else:
+            scores, new = d.batch_score_partial(ys, None if c["ids"] is None else t(c["ids"]), get(c["state"]), x)
+        np.testing.assert_allclose(scores.float().cpu().numpy(), rec[c["scores"]], rtol=2e-4, atol=2e-4, err_msg=what)
+        put(c["out"], new)
+    cw = decode_params(load(case)[0], dn)["ctc_weight"]
+    used = {c["scorer"] for c in log if c["op"] in ("score", "partial")}
+    assert used == {k for k, weight in (("decoder", 1.0 - cw), ("ctc", cw)) if weight}
 
 
 @pytest.mark.parametrize("dn", ["joint", "att", "ctc", "joint_pen"])
@@ -73,12 +92,11 @@ def test_reference_beam_search_drives_our_scorers_host_logic(dn, monkeypatch):
     import espnet_b200
     from gpu_util import refbuild
 
-    _reference()
     emu_backend.install_search(monkeypatch)
     z, cfg, w = load("tiny")
     model = espnet_b200.build_model(argparse.Namespace(**refbuild.model_yaml(cfg)))
     model.load_state_dict(w, strict=True)
-    _drive(model.eval(), z, dn, "cpu")
+    _replay(model.eval(), "tiny", dn, "cpu")
 
 
 @pytest.mark.gpu
@@ -87,10 +105,9 @@ def test_reference_beam_search_drives_our_scorers_host_logic(dn, monkeypatch):
 def test_reference_beam_search_drives_our_scorers_cuda(case, dn):
     from gpu_util import build_cuda_model
 
-    _reference()
     z, cfg, w = load(case)
     model, _ = build_cuda_model(cfg, w)
-    _drive(model, z, dn, "cuda")
+    _replay(model, case, dn, "cuda")
 
 
 @pytest.mark.gpu
